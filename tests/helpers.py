@@ -1,6 +1,7 @@
 """Shared test helpers: result comparison, the CPU unit-test driver for the product's
 __host__ __device__ functions (tests/host_core.cpp), reference device tables."""
 import ctypes as C
+import hashlib
 import json
 import os
 import subprocess
@@ -50,6 +51,55 @@ def compare_results(a, b, tag="", floats=True, stages=True):
                 d = np.nonzero(a[k] != b[k])[0] if len(a[k]) == len(b[k]) else []
                 diffs.append(f"{tag} stage {k} differs (len {len(a[k])} vs {len(b[k])}) first at {list(d[:3])}")
     return diffs
+
+
+def digest(obj):
+    """Short SHA-256 of an array (its bytes) or of a JSON-able value (numpy scalars as Python numbers)."""
+    if isinstance(obj, np.ndarray):
+        data = np.ascontiguousarray(obj).tobytes()
+    else:
+        data = json.dumps(obj, sort_keys=True, default=lambda v: v.item()).encode()
+    return hashlib.sha256(data).hexdigest()[:16]
+
+
+def fingerprint(res):
+    """A result dict in the compact, exact form tests/golden/reference.json stores: package headers in full, widths,
+    events and stage arrays as digests."""
+    fp = {"packages": [dict({k: p[k] for k in PKG_INT_KEYS + PKG_FLOAT_KEYS + ["depth_bits"]},
+                            widths=digest(np.concatenate([np.asarray(p["pulse"], np.int32), np.asarray(p["gap"], np.int32)])))
+                       for p in res["packages"]],
+          "events": len(res["events"]),
+          "events_digest": digest(np.array([(e["package"], e["dev"], e["hash"]) for e in res["events"]],
+                                           dtype=[("p", "<u4"), ("d", "<u4"), ("h", "<u8")]))}
+    for k in ("am", "fm"):
+        if k in res:
+            fp[k] = digest(np.asarray(res[k], np.int16))
+    return json.loads(json.dumps(fp, default=lambda v: v.item()))
+
+
+def compare_fingerprint(want, got, tag="", floats=True, stages=True):
+    """compare_results() for a recorded fingerprint `want` and a result dict `got`."""
+    g = fingerprint(got)
+    diffs = []
+    if len(want["packages"]) != len(g["packages"]):
+        diffs.append(f"{tag} package count {len(want['packages'])} != {len(g['packages'])}")
+    for i, (p, q) in enumerate(zip(want["packages"], g["packages"])):
+        for k in PKG_INT_KEYS + (PKG_FLOAT_KEYS + ["depth_bits"] if floats else []) + ["widths"]:
+            if p[k] != q[k]:
+                diffs.append(f"{tag} package {i} {k}: {p[k]} != {q[k]}")
+    if (want["events"], want["events_digest"]) != (g["events"], g["events_digest"]):
+        diffs.append(f"{tag} events differ: {want['events']} != {g['events']} or their digest")
+    if stages:
+        for k in ("am", "fm"):
+            if k in want and k in g and want[k] != g[k]:
+                diffs.append(f"{tag} stage {k} differs")
+    return diffs
+
+
+def events_digest(events):
+    """[count, digest] of a slicer's output: [(device index, bitbuffer record)]."""
+    return [len(events), digest(np.concatenate([np.frombuffer(np.uint32(d).tobytes() + bb.tobytes(), np.uint8)
+                                                for d, bb in events]) if events else np.zeros(0, np.uint8))]
 
 
 def default_devices():

@@ -6,6 +6,7 @@ import re
 
 import pytest
 
+import refdata
 from oracle import refh
 from rtl_433_b200 import lib
 
@@ -42,9 +43,8 @@ def test_no_oracle_in_product():
     assert "r433ref" not in out and "r433oracle" not in out
 
 
-@pytest.mark.skipif(not refh.available(), reason="oracle/_ref not built")
 def test_struct_layouts_match_reference():
-    facts = refh.abi_facts()
+    facts = refdata.recorded("abi_facts", refh.abi_facts)
     assert facts["sizeof_r_device"] == 152
     assert facts["sizeof_bitbuffer"] == 6604 == lib.BITBUFFER_DTYPE.itemsize
     assert facts["sizeof_pulse_data"] == 9672 == C.sizeof(lib.PulseData)

@@ -1,16 +1,16 @@
 """Pulse analyzer (SURVEY 8(f3)): r433b_analyze() -- histograms on the GPU (k_analyze), guess / RfRaw / text on the
 host, trial demodulation on the GPU (k_slice_own) -- against pulse_analyzer() of the compiled reference
-(src/pulse_analyzer.c:279-560): the stderr text, character for character, and the bitbuffers of the trial
-demodulation.  The histogram functions themselves are also run on the CPU through tests/host_core.cpp."""
+(src/pulse_analyzer.c:279-560; its answers recorded in tests/golden/reference.json by tests/refdata.py): the stderr
+text, character for character (as a digest), and the bitbuffers of the trial demodulation.  The histogram functions
+themselves are also run on the CPU through tests/host_core.cpp."""
 import random
 
 import numpy as np
 import pytest
 
-from oracle import refh
+import helpers
+import refdata
 from rtl_433_b200 import lib, synth
-
-needs_ref = pytest.mark.skipif(not refh.available(), reason="oracle/_ref/libr433ref.so not built")
 
 
 def shaped_package(rng, kind, rate=250000):
@@ -91,8 +91,23 @@ KINDS = ["single", "preamble", "ppm", "pwm_fixed_gap", "pwm_fixed_period", "manc
          "noclue", "many_bins", "fsk_zero_bin"]
 
 
+def analyzed_by_reference(key, ref, pd, package_type):
+    """[digest of pulse_analyzer()'s text, number and digest of the FNV-1a hashes of its trial demodulation's
+    bitbuffers]"""
+    def compute():
+        text, hashes = ref.analyze(pd, package_type)
+        return [helpers.digest(text), len(hashes), helpers.digest(hashes)]
+    return refdata.recorded(key, compute)
+
+
+def assert_analysis(want, text, bbs, what):
+    assert helpers.digest(text) == want[0], f"{what}: the analyzer's text differs from the reference's:\n{text}"
+    hashes = [fnv(bb) for bb in bbs]
+    assert [len(hashes), helpers.digest(hashes)] == want[1:], f"{what}: trial demodulation differs"
+
+
 def analyzer_matches_the_reference():
-    ref = refh.Ref(store_bitbuffers=False)
+    ref = refdata.LiveRef(store_bitbuffers=False)
     ctx = lib.Context(0)
     ctx.set_devices(lib.default_device_table()[:8])
     try:
@@ -115,10 +130,9 @@ def analyzer_matches_the_reference():
         for i, pd in enumerate(sent):
             k = res["packages"][i]
             assert int(k["num_pulses"]) == int(pd["num_pulses"])
-            want_text, want_hashes = ref.analyze(ctx_pulse_data(ctx, i), int(k["type"]))
+            want = analyzed_by_reference(f"analyzer/shaped/{i}", ref, ctx_pulse_data(ctx, i), int(k["type"]))
             a, g, text, bbs = ctx.analysis(i)
-            assert text == want_text, f"package {i}:\n--- reference\n{want_text}\n--- product\n{text}"
-            assert [fnv(bb) for bb in bbs] == want_hashes, f"package {i}: trial demodulation differs"
+            assert_analysis(want, text, bbs, f"package {i}")
             guesses.add(int(g.modulation))
         assert {0, 3, 4, 5, 6, 16, 17, 18} <= guesses, guesses
         ps.close()
@@ -131,10 +145,9 @@ def analyzer_matches_the_reference():
         assert res["n_packages"] >= 8
         demodulated = 0
         for i in range(res["n_packages"]):
-            want_text, want_hashes = ref.analyze(ctx_pulse_data(ctx, i), int(res["packages"][i]["type"]))
+            want = analyzed_by_reference(f"analyzer/capture/{i}", ref, ctx_pulse_data(ctx, i), int(res["packages"][i]["type"]))
             a, g, text, bbs = ctx.analysis(i)
-            assert text == want_text, f"capture package {i}"
-            assert [fnv(bb) for bb in bbs] == want_hashes
+            assert_analysis(want, text, bbs, f"capture package {i}")
             demodulated += len(bbs)
         assert demodulated >= 4
         y = synth.fsk_stream(7, n_samples=1 << 18, n_bursts=2).view(np.uint8)
@@ -143,10 +156,9 @@ def analyzer_matches_the_reference():
         ctx.analyze()
         assert any(int(t) == 2 for t in res["packages"]["type"])
         for i in range(res["n_packages"]):
-            want_text, want_hashes = ref.analyze(ctx_pulse_data(ctx, i), int(res["packages"][i]["type"]))
+            want = analyzed_by_reference(f"analyzer/fsk/{i}", ref, ctx_pulse_data(ctx, i), int(res["packages"][i]["type"]))
             a, g, text, bbs = ctx.analysis(i)
-            assert text == want_text, f"fsk package {i}"
-            assert [fnv(bb) for bb in bbs] == want_hashes
+            assert_analysis(want, text, bbs, f"fsk package {i}")
     finally:
         ref.close()
         ctx.close()
@@ -166,7 +178,6 @@ def fnv(bb):
 
 
 @pytest.mark.gpu
-@needs_ref
 def test_analyzer_matches_the_reference():
     analyzer_matches_the_reference()
 
@@ -175,8 +186,7 @@ def edge_cases_of_the_widening_rows():
     """Empty sets, a package without pulses, gates on loaded packages, call-order errors."""
     devices = lib.default_device_table()
     ctx = lib.Context(0)
-    ref = refh.Ref(store_bitbuffers=False)
-    ref.register_defaults()
+    ref = refdata.LiveRef(lambda r: r.register_defaults(), store_bitbuffers=False)
     try:
         ctx.set_devices(devices)
         ps = lib.Pulses()
@@ -190,21 +200,28 @@ def edge_cases_of_the_widening_rows():
         rng = random.Random(2)
         full = shaped_package(rng, "ppm")
         ps.add(full)
+        # without gates every event of the ppm package is the reference's, in order
+        ctx.process_pulses(ps)
+        ctx.fetch()
+        pd1 = ctx_pulse_data(ctx, 1)
+        want = [(e["dev"], e["hash"]) for e in helpers.gpu_stream_results(ctx, 0)["events"] if e["package"] == 1]
+
+        def sliced_by_reference():
+            ev = [[d, h] for d, h, _bb in ref.slice_pulse_data(pd1)]
+            return [len(ev), helpers.digest(ev)]
+        assert [len(want), helpers.digest(want)] == refdata.recorded("analyzer/edge/sliced", sliced_by_reference)
         ctx.set_gates(lib.default_gates(devices))
         ctx.process_pulses(ps)
         res = ctx.fetch()
         assert res["n_packages"] == 2
-        import helpers
         got = helpers.gpu_stream_results(ctx, 0)
-        want = ref.slice_pulse_data(ctx_pulse_data(ctx, 1))
         kept = [(e["dev"], e["hash"]) for e in got["events"] if e["package"] == 1]
         assert not [e for e in got["events"] if e["package"] == 0]
-        gates = lib.default_gates(devices)
         assert len(kept) + int(res["n_gated"]) == len(want) and res["n_gated"] > 0
         # the kept events are the reference's events the gates let through, in order
         it = iter(want)
         for dev, h in kept:
-            for d2, h2, _bb in it:
+            for d2, h2 in it:
                 if (d2, h2) == (dev, h):
                     break
             else:
@@ -212,9 +229,10 @@ def edge_cases_of_the_widening_rows():
         ctx.analyze()
         a, g, text, bbs = ctx.analysis(0)
         assert text == "No pulses detected.\n" and g.modulation == 0 and len(bbs) == 0
-        want_text, want_hashes = ref.analyze(ctx_pulse_data(ctx, 1), 1)
+        want = analyzed_by_reference("analyzer/edge/ppm", ref, pd1, 1)
         a, g, text, bbs = ctx.analysis(1)
-        assert text == want_text and [fnv(bb) for bb in bbs] == want_hashes and g.modulation == 5
+        assert_analysis(want, text, bbs, "ppm package")
+        assert g.modulation == 5
         ctx.set_gates(None)
         # call order: analyze needs a fetched batch
         x = synth.ook_stream(3, n_samples=1 << 17, n_bursts=1)
@@ -230,7 +248,6 @@ def edge_cases_of_the_widening_rows():
 
 
 @pytest.mark.gpu
-@needs_ref
 def test_edge_cases_of_the_widening_rows():
     edge_cases_of_the_widening_rows()
 
@@ -240,7 +257,7 @@ def analyzer_fuzz(n_packages=160, seed=31):
     B0 / B1 renderings, repeated groups, more than 32 groups, widths beyond 65535 us): text and trial demodulation
     against the reference."""
     rng = random.Random(seed)
-    ref = refh.Ref(store_bitbuffers=False)
+    ref = refdata.LiveRef(store_bitbuffers=False)
     ctx = lib.Context(0)
     ctx.set_devices([])
     try:
@@ -273,9 +290,9 @@ def analyzer_fuzz(n_packages=160, seed=31):
             a, g, text, bbs = ctx.analysis(i)
             if "this can't happen" in text:  # the reference exit(1)s there: the harness would not survive that package
                 continue
-            want_text, want_hashes = ref.analyze(ctx_pulse_data(ctx, i), int(res["packages"][i]["type"]))
-            assert text == want_text, f"package {i}:\n--- reference\n{want_text}\n--- product\n{text}"
-            assert [fnv(bb) for bb in bbs] == want_hashes, f"package {i}"
+            want = analyzed_by_reference(f"analyzer/fuzz/{seed}/{n_packages}/{i}", ref, ctx_pulse_data(ctx, i),
+                                         int(res["packages"][i]["type"]))
+            assert_analysis(want, text, bbs, f"package {i}")
             seen.add(int(g.modulation))
             if "+" in text.split("pdv/#")[-1].split("\n")[0]:
                 seen.add("b0-groups")
@@ -287,7 +304,6 @@ def analyzer_fuzz(n_packages=160, seed=31):
 
 
 @pytest.mark.gpu
-@needs_ref
 def test_analyzer_fuzz():
     analyzer_fuzz()
 

@@ -5,6 +5,7 @@ import os
 import numpy as np
 import pytest
 
+import refdata
 from oracle import orc, refh
 from rtl_433_b200 import captures, lib, synth
 
@@ -14,10 +15,9 @@ NAMES = ["g001_433.92M_250k.cu8", "x.cu8", "868M_1024k.cs16", "sdr_315M_1000k.cs
          "data_433.5M_3200k.cf32", "noext_250k_433M", "dir.v2/rec_1024K_868.35m.CS16", "9.cu8", "a_12345.cu8"]
 
 
-@pytest.mark.skipif(not refh.available(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", NAMES)
 def test_filename_metadata_matches_reference(name):
-    want = refh.parse_filename(name)
+    want = refdata.recorded(f"parse_filename/{name}", lambda: refh.parse_filename(name))
     got = captures.parse_capture_name(name)
     assert got["sample_rate"] == want["sample_rate"]
     assert got["center_frequency"] == want["center_frequency"]
@@ -84,7 +84,6 @@ def _make_sigmf(path, meta_name, meta, data, extra=()):
             tar.addfile(ti, io.BytesIO(payload))
 
 
-@pytest.mark.skipif(not refh.available(), reason="oracle/_ref not built")
 def test_sigmf_container_like_the_reference(tmp_path):
     """rate / frequency / start of the sample data as sigmf_reader_open() finds them (src/sigmf.c:336-434)."""
     x = synth.nice_flor_s_file()
@@ -100,7 +99,7 @@ def test_sigmf_container_like_the_reference(tmp_path):
     _make_sigmf(p2, "dir/a.sigmf-meta", m2, x.tobytes()[:1000], extra=[("dir/readme.txt", b"hello" * 300)])
     cases.append(p2)
     for p in cases:
-        want = refh.sigmf_open(p)
+        want = refdata.recorded(f"sigmf_open/{os.path.basename(p)}", lambda: refh.sigmf_open(p))
         got = captures.read_sigmf(p)
         assert want["rc"] == 0
         assert (got["sample_rate"], got["center_frequency"], got["data_offset"]) == (want["sample_rate"], want["center_frequency"], want["data_offset"])

@@ -1,7 +1,7 @@
 """CPU: the kernels' own source (k_detect, k_slice, k_cf32_to_cs16 and the C ABI around them) executed by
 the SIMT emulator (tests/emu.py, tests/simt/) under the SAME parity tests the GPU suite runs on the B200:
 every test function below is imported from the `-m gpu` modules and compares, through the C ABI, with the
-oracle (and the compiled reference).  Two lane schedules (ascending here, descending in
+oracle (and the recorded outputs of the compiled reference).  Two lane schedules (ascending here, descending in
 test_emu_reverse_schedule) catch a missing __syncwarp() in either direction."""
 import os
 
@@ -37,7 +37,6 @@ from test_gpu_parity import (ctx, devices,  # noqa: E402,F401  (fixtures)
 import test_pulse_io  # noqa: E402
 
 
-@test_pulse_io.needs_ref
 def test_emu_loaded_packages_through_k_slice():
     """r433b_process_pulses (SURVEY 8(f4)) under the emulator: the body of the -m gpu test."""
     test_pulse_io.loaded_packages_through_k_slice()
@@ -78,7 +77,6 @@ def test_emu_decoders_behind_gates_and_threads():
 import test_analyzer  # noqa: E402
 
 
-@test_analyzer.needs_ref
 def test_emu_analyzer_matches_the_reference():
     """k_analyze / k_slice_own (SURVEY 8(f3)) under the emulator: the body of the -m gpu test."""
     test_analyzer.analyzer_matches_the_reference()
@@ -110,12 +108,10 @@ def test_emu_slice_v1_still_exact(devices):
     assert subprocess.call([sys.executable, "-c", code], env=env) == 0
 
 
-@test_analyzer.needs_ref
 def test_emu_edge_cases_of_the_widening_rows():
     test_analyzer.edge_cases_of_the_widening_rows()
 
 
-@test_analyzer.needs_ref
 def test_emu_analyzer_fuzz():
     test_analyzer.analyzer_fuzz()
 

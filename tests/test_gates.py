@@ -1,7 +1,8 @@
 """Decoder length gates and the threaded replay (SURVEY 8(f1)).
 
 CPU: the committed gate table (rtl_433_b200/data/gates_25.12.json, tools/probe_gates.py) against the compiled
-reference decoders with inputs the generator never saw.  GPU / emulator: a gated run keeps exactly the events the
+reference decoders with inputs the generator never saw (their answers recorded in tests/golden/reference.json by
+tests/refdata.py).  GPU / emulator: a gated run keeps exactly the events the
 gate predicate lets through and counts the others per (package, device) and row class; with the reference's real
 decoders behind r433b_dispatch_r_devices() every decoder's statistics and the decoded messages are those of a
 pure-reference run -- gated or not, one thread or four."""
@@ -14,6 +15,7 @@ import numpy as np
 import pytest
 
 import helpers
+import refdata
 from oracle import refh
 from rtl_433_b200 import lib, synth
 
@@ -36,41 +38,61 @@ def all_protocols_ref():
     return L, r
 
 
-@needs_ref
-def test_gate_table_holds_for_fresh_inputs():
-    """A second probe with another seed never finds a shorter gate or another code than the committed table, and
-    hand-made bitbuffers below each gate (patterns the probe does not use) are turned down with the table's code."""
-    tab = gate_table()
+def probe_reference_decoders(tab):
+    """Per protocol: the gate a second probe (another seed) finds, its codes, and the distinct (single row, return
+    value, output count) answers of the decoder to 40 hand-made bitbuffers below the committed gate (patterns the
+    probe does not use: repeated rows and walking ones, what find_repeated_row() and preamble searches look for)."""
     L, r = all_protocols_ref()
-    devs = r.registered()
-    assert len(devs) == len(tab["gates"])
     rng = random.Random(99)
-    n_gated_devices = 0
-    for idx, d in enumerate(devs):
-        t, c1, cn = tab["gates"][str(d["protocol_num"])]
+    out = []
+    for idx, d in enumerate(r.registered()):
+        t = tab["gates"][str(d["protocol_num"])][0]
         code = (C.c_int * 2)()
         t2 = L.refh_probe_gate(r.h, idx, tab["max_bits"], 400, 12345, code)
-        assert t2 >= t, f"protocol {d['protocol_num']} {d['name']}: gate {t} does not hold (fresh probe: {t2})"
-        if t:
-            assert (code[0], code[1]) == (c1, cn)
-            n_gated_devices += 1
-        if t < 2:
-            continue
-        for k in range(40):
+        answers = set()
+        for k in range(40 if t >= 2 else 0):
             bb = np.zeros(1, refh.BITBUFFER_DTYPE)
             rows = 1 if k % 3 == 0 else rng.randrange(2, 30)
             bb["num_rows"] = rows
             bb["free_row"] = rows
             for row in range(rows):
                 bb["bits_per_row"][0][row] = rng.randrange(0, t)
-                # repeated rows and walking-ones: what find_repeated_row() and preamble searches look for
                 pat = [0xaa, 0x55, 0xff, 0x00, 0x2d, 0xd4, 0x80 >> (k % 8), rng.randrange(256)][k % 8]
                 bb["bb"][0][row][:4] = pat
-            out = C.c_int(0)
-            ret = L.refh_call_decoder(r.h, idx, bb.ctypes.data, C.byref(out))
-            assert ret == (c1 if rows == 1 else cn) and out.value == 0, (d["name"], rows, ret)
-    assert n_gated_devices > 300
+            n = C.c_int(0)
+            ret = L.refh_call_decoder(r.h, idx, bb.ctypes.data, C.byref(n))
+            answers.add((int(rows == 1), ret, n.value))
+        out.append({"protocol_num": d["protocol_num"], "gate": t, "probe": t2, "code": [code[0], code[1]],
+                    "answers": sorted(answers)})
     r.close()
+    return out
+
+
+def test_gate_table_holds_for_fresh_inputs():
+    """A second probe with another seed never finds a shorter gate or another code than the committed table, and
+    hand-made bitbuffers below each gate (patterns the probe does not use) are turned down with the table's code."""
+    tab = gate_table()
+    devs = lib.default_device_table(include_disabled=True)
+    n, want = refdata.registered_devices("all")
+    assert helpers.digest(refdata.device_rows(devs)) == want  # the reference's protocols in order
+    assert len(devs) == n == len(tab["gates"])
+    probed = refdata.recorded("gates/fresh_probe", lambda: probe_reference_decoders(tab))
+    assert [p["protocol_num"] for p in probed] == [d["protocol_num"] for d in devs]
+    n_gated_devices = 0
+    for d, p in zip(devs, probed):
+        t, c1, cn = tab["gates"][str(d["protocol_num"])]
+        assert p["gate"] == t, f"protocol {d['protocol_num']}: the gate table changed; record the probe again"
+        t2 = p["probe"]
+        assert t2 >= t, f"protocol {d['protocol_num']}: gate {t} does not hold (fresh probe: {t2})"
+        if t:
+            assert tuple(p["code"]) == (c1, cn)
+            n_gated_devices += 1
+        if t < 2:
+            continue
+        assert p["answers"]
+        for single, ret, n in p["answers"]:
+            assert ret == (c1 if single else cn) and n == 0, (d["protocol_num"], single, ret)
+    assert n_gated_devices > 300
 
 
 def gate_predicate(bb, t):

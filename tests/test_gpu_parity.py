@@ -1,7 +1,7 @@
 """-m gpu: the CUDA path (through the C ABI) against the oracle on the same seeded inputs.
 
-Oracle = oracle/r433_oracle.c (CPU restatement) and, when the prebuilt file travelled with the
-snapshot, oracle/_ref/libr433ref.so (the unmodified reference).  Everything integer is compared
+Oracle = oracle/r433_oracle.c (CPU restatement) and the unmodified reference (oracle/_ref/libr433ref.so, its
+outputs recorded in tests/golden/reference.json by tests/refdata.py).  Everything integer is compared
 for equality: stage arrays, pulse widths, package headers, every bitbuffer (by FNV-1a of the
 whole 6604-byte struct) in the reference's dispatch order.  The only floats on the path
 (calc_rssi_snr, src/r_flow.c:35-64) are computed on the host with the reference's expressions and
@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 import helpers
+import refdata
 from oracle import orc, refh
 from rtl_433_b200 import lib, synth
 
@@ -142,19 +143,20 @@ def test_fm_rebuild_after_constant_input(ctx, devices):
         check(gpu[i], ref, f"constant cs16 {i}")
 
 
+def check_recorded(gpu, want, tag):
+    d = helpers.compare_fingerprint(want, gpu, tag)
+    assert not d, "\n".join(d[:20])
+
+
 def test_against_compiled_reference(ctx, devices):
-    """Same comparison against the unmodified reference when oracle/_ref travelled here."""
-    if not refh.available():
-        pytest.skip("oracle/_ref/libr433ref.so not present")
-    r = refh.Ref(store_bitbuffers=False, store_stages=True)
-    r.register_defaults()
+    """Same comparison against the unmodified reference."""
     streams = [synth.ook_stream(100 + seed) for seed in range(2)]
     gpu = run_gpu(ctx, streams, lib.FMT_CU8, 250000, 433920000)
     for i, s in enumerate(streams):
-        check(gpu[i], r.run(s, 2), f"ref ook {i}")
+        check_recorded(gpu[i], refdata.ref_run(f"gpu_parity/ook/{i}", s, 2), f"ref ook {i}")
     streams = [synth.fsk_stream(100)]
     gpu = run_gpu(ctx, streams, lib.FMT_CS16, 1024000, 868000000)
-    check(gpu[0], r.run(streams[0], 4, 1024000, 868000000, 2), "ref fsk")
+    check_recorded(gpu[0], refdata.ref_run("gpu_parity/fsk", streams[0], 4, 1024000, 868000000, 2), "ref fsk")
 
 
 def test_ragged_lengths_and_small_blocks(ctx, devices):

@@ -1,9 +1,9 @@
 """Pulse-level I/O (SURVEY 8(f4)): `.ook` / RfRaw readers and `.ook` / VCD / logic.u8 writers of the product
-(host functions of libr433b.so, rtl_433_b200/csrc/r433b_pulses.hpp) against the compiled reference
-(pulse_data_load, rfraw_parse, pulse_data_dump, pulse_data_print_vcd, pulse_data_dump_raw of oracle/_ref) and
-against the committed golden fixture (tests/golden/pulse_io.json, generated from the reference by
-tools/make_golden.py).  The -m gpu part sends loaded packages through k_slice and compares every bitbuffer
-with run_ook_demods() / run_fsk_demods() of the reference on the same pulse_data_t."""
+(host functions of libr433b.so, rtl_433_b200/csrc/r433b_pulses.hpp) against the reference (what pulse_data_load,
+rfraw_parse, pulse_data_dump, pulse_data_print_vcd and pulse_data_dump_raw of oracle/_ref return, recorded in
+tests/golden/reference.json by tests/refdata.py) and against the committed golden fixture (tests/golden/pulse_io.json,
+generated from the reference by tools/make_golden.py).  The -m gpu part sends loaded packages through k_slice and
+compares every bitbuffer with run_ook_demods() / run_fsk_demods() of the reference on the same pulse_data_t."""
 import json
 import os
 import random
@@ -12,13 +12,12 @@ import numpy as np
 import pytest
 
 import helpers
+import refdata
 from oracle import refh
 from rtl_433_b200 import lib, synth
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLDEN = os.path.join(HERE, "golden", "pulse_io.json")
-
-needs_ref = pytest.mark.skipif(not refh.available(), reason="oracle/_ref/libr433ref.so not built")
 
 INT_FIELDS = ["sample_rate", "num_pulses", "fsk_f1_est", "fsk_f2_est", "offset", "depth_bits", "start_ago", "end_ago",
               "ook_low_estimate", "ook_high_estimate"]
@@ -118,25 +117,32 @@ def random_pulse_data(rng, fsk=False):
     return pd
 
 
-@needs_ref
+def ref_loaded(key, text, rate, cap=64):
+    """digest of what pulse_data_load() reads out of `text`."""
+    return refdata.recorded(key, lambda: helpers.digest([pd_facts(p) for p in refh.load_ook(text, rate, cap=cap)]))
+
+
 def test_ook_and_rfraw_readers_match_the_reference():
     for name, text in ook_cases().items():
         for rate in RATES:
-            want = [pd_facts(p) for p in refh.load_ook(text, rate, cap=64)]
             got = product_load(text, rate)
-            assert got == want, f"case {name} @ {rate}"
+            assert helpers.digest(got) == ref_loaded(f"pulse_io/load/{name}/{rate}", text, rate), f"case {name} @ {rate}"
     # the -y test-data path: rfraw_parse() into a zeroed struct
     ps = lib.Pulses()
     for name, text in ook_cases().items():
         if not name.startswith("rfraw"):
             continue
         line = text.split("\n")[0]
-        ref = refh.rfraw(line)
+
+        def ref_rfraw():
+            ref = refh.rfraw(line)
+            return None if ref is None else helpers.digest(pd_facts(ref))
+        ref = refdata.recorded(f"pulse_io/rfraw/{name}", ref_rfraw)
         ps.clear()
         n = ps.load_rfraw(line)
         assert n == (1 if ref is not None else 0), name
         if n:
-            assert pd_facts(ps.get(0)) == pd_facts(ref), name
+            assert helpers.digest(pd_facts(ps.get(0))) == ref, name
     assert ps.load_rfraw("500 1000") == 0
     ps.close()
 
@@ -167,45 +173,50 @@ def random_ook_text(rng):
     return rng.choice(["\n", "\r\n"]).join(lines) + rng.choice(["\n", ""])
 
 
-@needs_ref
 def test_ook_reader_random_texts():
     """400 random pulse texts (rows, headers, whole / truncated / decorated RfRaw lines, junk): the same packages as
     pulse_data_load() reads out of them."""
+    cases = []
     for seed in range(400):
         rng = random.Random(1000 + seed)
         text = random_ook_text(rng)
-        rate = rng.choice(RATES)
-        want = [pd_facts(p) for p in refh.load_ook(text, rate, cap=128)]
-        assert product_load(text, rate) == want, f"seed {seed}: {text!r}"
+        cases.append((text, rng.choice(RATES)))
+    want = refdata.recorded("pulse_io/random_texts", lambda: [helpers.digest([pd_facts(p) for p in refh.load_ook(text, rate, cap=128)])
+                                                              for text, rate in cases])
+    for seed, (text, rate) in enumerate(cases):
+        assert helpers.digest(product_load(text, rate)) == want[seed], f"seed {seed}: {text!r}"
 
 
-@needs_ref
 def test_writers_match_the_reference():
     rng = random.Random(11)
     for i in range(40):
         pd = random_pulse_data(rng, fsk=i % 3 == 0)
-        ref = refh.dump_ook(pd)
-        assert ref.startswith(";received ")
-        assert lib.format_ook(pd) == ref[ref.index("\n") + 1:]
-        assert lib.format_ook(pd, received="@1.5s") == ";received @1.5s\n" + ref[ref.index("\n") + 1:]
-        for ch in "'\"":
-            assert lib.format_vcd(pd, ch) == refh.dump_vcd(pd, ch)
-        head = refh.dump_vcd(pd, "'", header=True)
-        body = refh.dump_vcd(pd, "'")
-        ref_head = head[:len(head) - len(body)]
-        date = ref_head.split("\n")[0][len("$date "):-len(" $end")]
-        assert lib.format_vcd_header(int(pd["sample_rate"]), date) == ref_head
         # logic.u8: a window that cuts the package at both ends
         total = int(pd["pulse"][:pd["num_pulses"]].sum() + pd["gap"][:pd["num_pulses"]].sum())
         start = int(pd["offset"]) + total // 4 if i % 2 else max(0, int(pd["offset"]) - 100)
         length = max(1, min(total // 2 + 7, 200000))
         bits = 0x04 if pd["fsk_f2_est"] else 0x02
-        assert np.array_equal(lib.dump_logic_u8(pd, length, start, bits), refh.dump_raw(pd, length, start, bits))
+
+        def written():
+            ref = refh.dump_ook(pd)
+            assert ref.startswith(";received ")
+            head = refh.dump_vcd(pd, "'", header=True)
+            body = refh.dump_vcd(pd, "'")
+            ref_head = head[:len(head) - len(body)]
+            return {"ook": helpers.digest(ref[ref.index("\n") + 1:]), "vcd": [helpers.digest(refh.dump_vcd(pd, ch)) for ch in "'\""],
+                    "date": ref_head.split("\n")[0][len("$date "):-len(" $end")], "vcd_header": helpers.digest(ref_head),
+                    "logic_u8": helpers.digest(refh.dump_raw(pd, length, start, bits))}
+        ref = refdata.recorded(f"pulse_io/writers/{i}", written)
+        assert helpers.digest(lib.format_ook(pd)) == ref["ook"]
+        assert lib.format_ook(pd, received="@1.5s").startswith(";received @1.5s\n")
+        assert helpers.digest(lib.format_ook(pd, received="@1.5s")[len(";received @1.5s\n"):]) == ref["ook"]
+        assert [helpers.digest(lib.format_vcd(pd, ch)) for ch in "'\""] == ref["vcd"]
+        assert helpers.digest(lib.format_vcd_header(int(pd["sample_rate"]), ref["date"])) == ref["vcd_header"]
+        assert helpers.digest(lib.dump_logic_u8(pd, length, start, bits)) == ref["logic_u8"]
     assert lib.format_ook_header() == ";pulse data\n;version 1\n;timescale 1us\n"
     assert lib.format_ook_header("now") == ";pulse data\n;version 1\n;timescale 1us\n;created now\n"
 
 
-@needs_ref
 def test_dump_then_load_round_trip_like_the_reference():
     """pulse_data_dump() rounds to whole microseconds; loading that text back must give what the reference loads."""
     rng = random.Random(5)
@@ -214,7 +225,7 @@ def test_dump_then_load_round_trip_like_the_reference():
     for pd in pds:
         text += lib.format_ook(pd, received="t")
     for rate in RATES:
-        assert product_load(text, rate) == [pd_facts(p) for p in refh.load_ook(text, rate)]
+        assert helpers.digest(product_load(text, rate)) == ref_loaded(f"pulse_io/round_trip/{rate}", text, rate)
     assert len(product_load(text, 250000)) == len(pds)
 
 
@@ -244,7 +255,6 @@ def sliced_by_reference(ref, pd):
 
 
 @pytest.mark.gpu
-@needs_ref
 def test_loaded_packages_through_k_slice():
     """`.ook` text and RfRaw lines -> r433b_process_pulses -> every bitbuffer equal to the reference's slicers."""
     loaded_packages_through_k_slice()
@@ -254,8 +264,7 @@ def loaded_packages_through_k_slice():
     devices = lib.default_device_table()
     ctx = lib.Context(0)
     ctx.set_devices(devices)
-    ref = refh.Ref(store_bitbuffers=False)
-    ref.register_defaults()
+    ref = refdata.LiveRef(lambda r: r.register_defaults(), store_bitbuffers=False)
     try:
         # packages k_detect finds in two synthetic captures, written as .ook text by the product
         x = [synth.ook_stream(s, n_samples=1 << 19, n_bursts=4) for s in (21, 22)]
@@ -300,10 +309,16 @@ def loaded_packages_through_k_slice():
         ps.add(fsk_pd, stream=3)
         ps.add(random_pulse_data(rng), stream=3)
 
-        want_sets = [list(refh.load_ook(texts[0], 250000)), list(refh.load_ook(texts[1], 250000)),
-                     list(refh.load_ook(mixed, 1024000)), [refh.rfraw(cases["rfraw_b1_line"].strip()), fsk_pd, ps.get(len(ps) - 1)]]
+        def loaded_by_reference():
+            sets = [list(refh.load_ook(texts[0], 250000)), list(refh.load_ook(texts[1], 250000)),
+                    list(refh.load_ook(mixed, 1024000)), [refh.rfraw(cases["rfraw_b1_line"].strip()), fsk_pd, ps.get(len(ps) - 1)]]
+            return [[{"num_pulses": int(p["num_pulses"]), "sample_rate": int(p["sample_rate"]),
+                      "pulse": helpers.digest(p["pulse"][:int(p["num_pulses"])]), "freq1_hz": float(p["freq1_hz"]),
+                      "fsk_f2_est": int(p["fsk_f2_est"]), "events": helpers.digest(sliced_by_reference(ref, p))} for p in w]
+                    for w in sets]
+        want_sets = refdata.recorded("pulse_io/loaded_through_k_slice", loaded_by_reference)
         assert sum(len(w) for w in want_sets) == len(ps)
-        assert len({int(p["sample_rate"]) for w in want_sets for p in w}) >= 3
+        assert len({p["sample_rate"] for w in want_sets for p in w}) >= 3
 
         ctx.process_pulses(ps)
         ctx.fetch()
@@ -312,12 +327,11 @@ def loaded_packages_through_k_slice():
             got = helpers.gpu_stream_results(ctx, s)
             assert len(got["packages"]) == len(want)
             for li, (gp, wp) in enumerate(zip(got["packages"], want)):
-                assert gp["num_pulses"] == int(wp["num_pulses"]) and gp["sample_rate"] == int(wp["sample_rate"])
-                assert np.array_equal(gp["pulse"][:gp["num_pulses"]], wp["pulse"][:gp["num_pulses"]])
-                assert gp["freq1_hz"] == float(wp["freq1_hz"]) and gp["fsk_f2_est"] == int(wp["fsk_f2_est"])
+                assert gp["num_pulses"] == wp["num_pulses"] and gp["sample_rate"] == wp["sample_rate"]
+                assert helpers.digest(gp["pulse"][:gp["num_pulses"]].astype(np.int32)) == wp["pulse"]
+                assert gp["freq1_hz"] == wp["freq1_hz"] and gp["fsk_f2_est"] == wp["fsk_f2_est"]
                 mine = [(e["dev"], e["hash"]) for e in got["events"] if e["package"] == li]
-                theirs = sliced_by_reference(ref, wp)
-                assert mine == theirs, f"stream {s} package {li}: {len(mine)} vs {len(theirs)} events"
+                assert helpers.digest(mine) == wp["events"], f"stream {s} package {li}: {len(mine)} events differ from the reference's"
                 total_events += len(mine)
         assert total_events > 1000
         assert ctx.counts()["events"] == total_events
